@@ -5,6 +5,7 @@ reference algorithm's CPU timing.
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload timesformer|vivit|mvit|maskfeat] [--batch B]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference [--steps K --warmup W]      # CPU arm (oracle port of the reference)
+    python bench.py --dump-outputs DIR ...                       # also write the last timed step's outputs as DIR/*.npy
 
 One JSON line on stdout (rank 0).  Workloads = BASELINE.json configs:
   timesformer (default, configs 1-2)  TimeSformer-B divided_space_time 8x224x224, batch 8 / GPU, + cls head + CE
@@ -19,6 +20,12 @@ gradient all-reduce.  The optimizer update is outside the metric (BASELINE.json:
           maskfeat: the uint8 clips; masks drawn on the host, HOG targets computed on the device inside the region) and the
           loss read back to the host
 The default line also carries `other_workloads`: the same measurement for the three other configs.
+--dump-outputs DIR writes what the caller of the timed step receives after its last timed step: the loss (loss.npy) and
+every parameter gradient (grad.<parameter name>.npy, float32; a gradient of more than DUMP_SAMPLE elements as the same
+seeded sample of its flattened elements on every run).  Inputs, weights and DropPath draws are seeded, so two builds run
+with the same arguments can be compared array for array.  Split-K GEMMs add their partial sums in an order that varies
+from run to run, and the bf16 operand casts downstream can turn such last-bit differences into bf16-rounding ones: compare
+gradients with a tolerance, not bit for bit.  The benchmark writes nothing into the source tree.
 """
 from __future__ import annotations
 
@@ -36,6 +43,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: no __pycache__ written into it
 
 UNIT = 'clips/s'
 IMG, NUM_CLASSES = 224, 400
@@ -50,6 +58,7 @@ WORKLOADS = {
     'maskfeat': dict(metric='clips/sec (BxTx3x224x224) MaskFeat MViT-B pretrain fwd+bwd', frames=16, batch=16, flop_per_clip=0.516e12,
                      desc='MaskFeat MViT-B pretrain step 16x224x224: cube masks, HOG targets (HOG kernel), decoder + masked MSE, fwd+bwd'),
 }
+DUMP_SAMPLE, DUMP_MAX_BYTES = 1 << 16, 64 << 20
 # attention-GEMM subset of the TimeSformer step (north_star): qkv + QK^T + PV + out-proj of both passes, fwd+bwd
 MASKFEAT_KW = dict(pool_q_stride_size=[[1, 1, 2, 2], [3, 1, 2, 2]], feature_dim=2 * 2 * 2 * 3 * 9)
 
@@ -317,8 +326,31 @@ class WorkloadRun:
         return x, target, mask, cmask
 
 
-def measure(run, args, world, rank, dist, steps, with_probe):
-    """Times one workload: graph-captured step (value), e2e through host buffers, optional GEMM / attention probe."""
+def dump_outputs(net, loss, out_dir):
+    """loss.npy and grad.<name>.npy for every parameter with a gradient; see --dump-outputs in the module docstring."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {'loss': loss.detach().reshape(1)}
+    for n, p in net.named_parameters():
+        if p.grad is None:
+            continue
+        g = p.grad.detach().reshape(-1)
+        if g.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(g.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            g = g[idx.to(g.device)]
+        arrays['grad.' + n] = g
+    total = sum(a.numel() * (8 if a.dtype == torch.float64 else 4) for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f'--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte budget')
+    for n, a in arrays.items():
+        a = a.cpu()
+        np.save(os.path.join(out_dir, n + '.npy'), a.numpy() if a.dtype == torch.float64 else a.float().numpy())
+    return {'dir': out_dir, 'arrays': len(arrays), 'bytes': total}
+
+
+def measure(run, args, world, rank, dist, steps, with_probe, dump_dir=None):
+    """Times one workload: graph-captured step (value), e2e through host buffers, optional GEMM / attention probe;
+    with dump_dir, writes the outputs of the last timed step there (dump_outputs)."""
     from videotransformer_pytorch_b200 import _lib
     from videotransformer_pytorch_b200.ddp import GradientBuckets
     from videotransformer_pytorch_b200.graph import GraphedTrainStep
@@ -370,12 +402,17 @@ def measure(run, args, world, rank, dist, steps, with_probe):
     for _ in range(max(args.warmup, 3)):
         loss = step(*step_inputs)
     barrier()
+    last = {}
+
+    def timed_step():
+        last['loss'] = step(*step_inputs)
     l0 = _lib.launch_count()
-    ms_dev = timed(lambda: step(*step_inputs), steps)
+    ms_dev = timed(timed_step, steps)
     launches = (_lib.launch_count() - l0)
     if graphed is not None:      # replays launch the kernels recorded at capture time (the host-side counter is not touched)
         launches = graphed.kernels_per_replay * steps
     loss_value = float(loss.item())
+    dumped = dump_outputs(net, last['loss'], dump_dir) if dump_dir else None
 
     # End to end through the public API: every step's batch comes from pinned host memory and the loss goes back to the
     # host.  The copy of step i+1 is issued on a copy stream while step i computes (double-buffered device staging),
@@ -409,7 +446,7 @@ def measure(run, args, world, rank, dist, steps, with_probe):
     e2e_step()
     ms_e2e = timed(e2e_step, steps)
 
-    res = dict(ms_dev=ms_dev, ms_e2e=ms_e2e, launches=launches, loss=loss_value, reducer=reducer, graphed=graphed,
+    res = dict(ms_dev=ms_dev, ms_e2e=ms_e2e, launches=launches, loss=loss_value, dumped=dumped, reducer=reducer, graphed=graphed,
                step_inputs=step_inputs, eager_step=eager_step, kernels_per_replay=(graphed.kernels_per_replay if graphed else None))
     if with_probe:
         try:
@@ -599,7 +636,8 @@ def main_gpu(args):
     B = args.batch or w['batch']
     run = WorkloadRun(name, dev, B, rank)
     sampler = ClockSampler(torch.cuda.current_device()) if rank == 0 else None
-    res = measure(run, args, world, rank, dist, args.steps, with_probe=True)
+    res = measure(run, args, world, rank, dist, args.steps, with_probe=True,
+                  dump_dir=args.dump_outputs if rank == 0 else None)
     clocks = sampler.stop() if sampler else None
     check = None
     if world > 1:
@@ -704,6 +742,8 @@ def main_gpu(args):
             line['exchange'] = exposed
         if others:
             line['other_workloads'] = others
+        if res['dumped'] is not None:
+            line['dumped_outputs'] = res['dumped']
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -728,7 +768,11 @@ def main():
     ap.add_argument('--no-graph', action='store_true', help='issue the step kernel by kernel instead of replaying a CUDA graph')
     ap.add_argument('--no-others', dest='others', action='store_false', help='skip the other BASELINE configs in the default line')
     ap.add_argument('--no-baselines', dest='baselines', action='store_false', help='skip the CPU / eager-GPU comparators (A/B runs)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the loss and parameter gradients of the last timed step '
+                                                          'to DIR/<name>.npy (gradients sampled: see the module docstring)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         return main_reference(args)
     if int(os.environ.get('WORLD_SIZE', '1')) > 1 or args.workload != 'timesformer':

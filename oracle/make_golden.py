@@ -8,7 +8,7 @@ The reference is imported unmodified with `sys.modules` stubs for its
 non-arithmetic top-level imports (matplotlib, pytorch_lightning.utilities.distributed,
 pytorchvideo.* — SURVEY.md §8c).  For every case the script also runs the oracle
 restatement (oracle/vt_oracle.py, oracle/mask_oracle.py) and asserts agreement,
-i.e. this script is what pins the oracle.  Outputs are small .npz files.
+i.e. this script is what pins the oracle.  Outputs are small .npz / .json files.
 """
 from __future__ import annotations
 
@@ -16,6 +16,7 @@ import hashlib
 import os
 import random
 import sys
+import tempfile
 import types
 
 import numpy as np
@@ -423,6 +424,105 @@ def mixup_cases():
     print(f'[mixup] {len(seeds)} seeds stored from the reference Mixup class')
 
 
+def checkpoint_remap_cases():
+    """The reference's pretrain_pth loaders (weight_init.py:107-314) on the synthetic checkpoints of
+    tests/test_checkpoint_loaders.py: per case the key set of the state dict handed to load_state_dict and, per key, the
+    shape and a SHA-256 prefix of the tensor bytes (the remaps are copies / repeats / scalings, compared bit for bit)."""
+    import json
+    from tests import test_checkpoint_loaders as T
+    sys.path.insert(0, REF)
+    import weight_init as ref_wi
+
+    class Catch(torch.nn.Module):
+        """stands in for the model: records the state dict the reference loader hands to load_state_dict"""
+        def load_state_dict(self, sd, strict=True):
+            self.got = dict(sd)
+            return torch.nn.modules.module._IncompatibleKeys([], [])
+
+    rows = {}
+    with tempfile.TemporaryDirectory() as d:
+        for conv_type, attention_type, copy_strategy, extend in T.REMAP_CASES:
+            for kind, make, ref_fn, inner in (('vit', T._vit_image_checkpoint, ref_wi.init_from_vit_pretrain_, 'state_dict'),
+                                              ('mae', T._mae_checkpoint, ref_wi.init_from_mae_pretrain_, 'model')):
+                path = os.path.join(d, f'{kind}.pth')
+                torch.save({inner: make()}, path)
+                catch = Catch()
+                ref_fn(catch, path, conv_type, attention_type, copy_strategy, extend, 2, 1)
+                rows[T.remap_case_id(kind, conv_type, attention_type, copy_strategy, extend)] = T.state_digest(catch.got)
+    sd = T._kinetics_checkpoint()
+    ref_wi.replace_state_dict(sd)
+    rows['kinetics'] = T.state_digest(sd)
+    with open(os.path.join(GOLD, 'checkpoint_remaps.json'), 'w') as fh:          # one line per case
+        fh.write('{\n' + ',\n'.join(f'{json.dumps(c)}: {json.dumps(rows[c], sort_keys=True)}' for c in sorted(rows)) + '\n}\n')
+    print(f'[checkpoint_remaps] {len(rows)} state dicts from the reference loaders')
+
+
+def trainer_case():
+    """What the reference's model_trainer.py asks of the modules videotransformer_pytorch_b200/shim stands in for: the
+    names the reference files import from them, the constructor calls VideoTransformer.__init__ (model_trainer.py:40-104)
+    makes for one supervised TimeSformer configuration, and the parameter names / shapes and no-weight-decay keywords of
+    the trainer built from the reference's own modules."""
+    import ast
+    import importlib
+    import json
+    from tests.test_shim import SHIM, SHIM_MODULES, TRAINER_CFG
+
+    def stub(name, **attrs):
+        m = types.ModuleType(name)
+        m.__dict__.update(attrs)
+        sys.modules[name] = m
+
+    class Accuracy:
+        def __init__(self, *a, **k):
+            pass
+
+    stub('pytorch_lightning', LightningModule=torch.nn.Module)
+    stub('pytorch_lightning.utilities')
+    stub('pytorch_lightning.utilities.distributed', rank_zero_only=lambda f: f)
+    stub('torchmetrics', Accuracy=Accuracy)
+    stub('timm'); stub('timm.loss', SoftTargetCrossEntropy=torch.nn.CrossEntropyLoss)
+    stub('matplotlib'); stub('matplotlib.pyplot')
+    from oracle.pytorchvideo_restated import install_stub_modules
+    install_stub_modules()
+    imports = {}
+    for f in sorted(os.listdir(REF)):
+        if f.endswith('.py'):
+            with open(os.path.join(REF, f)) as fh:
+                for node in ast.walk(ast.parse(fh.read())):
+                    if isinstance(node, ast.ImportFrom) and node.level == 0 and node.module in SHIM_MODULES:
+                        imports.setdefault(node.module, set()).update(a.name for a in node.names)
+    cfg = types.SimpleNamespace(**TRAINER_CFG)
+    saved_path = list(sys.path)
+
+    def fresh_trainer(first):
+        for k in SHIM_MODULES + ('model_trainer', 'utils', 'optimizer', 'weight_init'):
+            sys.modules.pop(k, None)
+        sys.path[:] = first + [REF] + saved_path
+        return importlib.import_module('model_trainer')
+
+    # with the shim first on sys.path: record every model / head constructor call the trainer makes
+    calls = []
+    fresh_trainer([SHIM])
+    for mod, name in (('video_transformer', 'TimeSformer'), ('video_transformer', 'ViViT'), ('video_transformer', 'MaskFeat'),
+                      ('transformer', 'ClassificationHead')):
+        cls = getattr(sys.modules[mod], name)
+        setattr(sys.modules[mod], name, lambda *a, _n=name, _c=cls, **k: calls.append([_n, list(a), k]) or _c(*a, **k))
+    sys.modules.pop('model_trainer')
+    importlib.import_module('model_trainer').VideoTransformer(cfg, trainer=None, ckpt_dir='.', do_eval=False, do_test=False)
+    # the reference's own modules: the parameter surface the trainer (and its optimizer grouping) sees
+    torch.manual_seed(0)
+    vt_ref = fresh_trainer([]).VideoTransformer(cfg, trainer=None, ckpt_dir='.', do_eval=False, do_test=False)
+    sys.path[:] = saved_path
+    row = {'cfg': TRAINER_CFG, 'imports': {k: sorted(v) for k, v in sorted(imports.items())}, 'constructions': calls,
+           'named_parameters': [[n, list(p.shape)] for n, p in vt_ref.named_parameters()],
+           'no_weight_decay_keywords': sorted(vt_ref.no_weight_decay_keywords())}
+    with open(os.path.join(GOLD, 'reference_trainer.json'), 'w') as fh:          # one line per entry / parameter
+        fh.write('{\n' + ',\n'.join(f'{json.dumps(k)}: ' + ('[\n' + ',\n'.join(json.dumps(e) for e in v) + '\n]'
+                                                            if k == 'named_parameters' else json.dumps(v))
+                                     for k, v in row.items()) + '\n}\n')
+    print(f'[reference_trainer] {len(calls)} constructor calls, {len(row["named_parameters"])} parameters')
+
+
 def main_selected(tr, vt, mg, only):
     """Cases added after round 1 (run alone with `python oracle/make_golden.py <name> ...`)."""
     want = lambda n: only is None or n in only
@@ -438,6 +538,10 @@ def main_selected(tr, vt, mg, only):
         vivit_variant_case(vt, 'vivit_divided_hd64', vv128, B=2, seed=14, attention_type='divided_space_time')
     if want('mixup'):
         mixup_cases()
+    if want('checkpoint_remaps'):
+        checkpoint_remap_cases()
+    if want('reference_trainer'):
+        trainer_case()
 
 
 if __name__ == '__main__':

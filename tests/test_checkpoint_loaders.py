@@ -1,16 +1,37 @@
 """pretrain_pth checkpoint loaders (weight_init.py) against the reference's own functions (weight_init.py:107-314).
 
-The reference is importable only in the build container (/root/reference); there the remapped state dicts are compared
-key by key and value by value.  Everywhere, the constructors' `pretrain_pth` flow is exercised with a synthetic checkpoint
-(ADVICE r1: the drop-in claim must hold for the reference's standard finetune flow)."""
+The remapped state dicts of synthetic checkpoints are compared key by key and bit for bit with what the reference loaders
+produced from the same checkpoints (tests/golden/checkpoint_remaps.json, written by `oracle/make_golden.py
+checkpoint_remaps`).  The constructors' `pretrain_pth` flow is exercised with a synthetic checkpoint as well: the drop-in
+claim must hold for the reference's standard finetune flow."""
+import hashlib
+import json
 import os
-import sys
-import types
 
 import pytest
 import torch
 
-REF = '/root/reference'
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'checkpoint_remaps.json')
+REMAP_CASES = [
+    ('Conv2d', 'divided_space_time', 'repeat', 'temporal_avg'), ('Conv2d', 'space_only', 'repeat', 'temporal_avg'),
+    ('Conv3d', 'fact_encoder', 'repeat', 'temporal_avg'), ('Conv3d', 'fact_encoder', 'set_zero', 'center_frame'),
+    ('Conv3d', 'joint_space_time', 'repeat', 'center_frame'), ('Conv2d', 'divided_space_time', 'set_zero', 'temporal_avg')]
+
+
+def remap_case_id(kind, *case):
+    return '/'.join((kind,) + case)
+
+
+def state_digest(sd):
+    """key -> [dtype, shape, SHA-256 prefix of the contiguous tensor bytes]"""
+    return {k: [str(v.dtype), list(v.shape), hashlib.sha256(v.detach().contiguous().numpy().tobytes()).hexdigest()[:16]]
+            for k, v in sd.items()}
+
+
+@pytest.fixture(scope='module')
+def reference_remaps():
+    with open(GOLDEN) as fh:
+        return json.load(fh)
 
 
 def _vit_image_checkpoint(D=32, L=2, P=4):
@@ -48,56 +69,28 @@ def _mae_checkpoint(D=32, L=2):
     return sd
 
 
-def _reference_weight_init():
-    if not os.path.isdir(REF):
-        pytest.skip('/root/reference not present (build container only)')
-    for name in ('matplotlib', 'matplotlib.pyplot', 'pytorch_lightning', 'pytorch_lightning.utilities'):
-        sys.modules.setdefault(name, types.ModuleType(name))
-    m = types.ModuleType('pytorch_lightning.utilities.distributed')
-    m.rank_zero_only = lambda f: f
-    sys.modules.setdefault('pytorch_lightning.utilities.distributed', m)
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    import importlib
-    return importlib.import_module('weight_init')
-
-
-class _Catch(torch.nn.Module):
-    """stands in for the model: records the state dict the reference loader hands to load_state_dict"""
-    def load_state_dict(self, sd, strict=True):
-        self.got = dict(sd)
-        return torch.nn.modules.module._IncompatibleKeys([], [])
-
-
-@pytest.mark.parametrize('conv_type,attention_type,copy_strategy,extend', [
-    ('Conv2d', 'divided_space_time', 'repeat', 'temporal_avg'), ('Conv2d', 'space_only', 'repeat', 'temporal_avg'),
-    ('Conv3d', 'fact_encoder', 'repeat', 'temporal_avg'), ('Conv3d', 'fact_encoder', 'set_zero', 'center_frame'),
-    ('Conv3d', 'joint_space_time', 'repeat', 'center_frame'), ('Conv2d', 'divided_space_time', 'set_zero', 'temporal_avg')])
-def test_vit_and_mae_remaps_equal_the_reference(tmp_path, conv_type, attention_type, copy_strategy, extend):
-    ref = _reference_weight_init()
-    from videotransformer_pytorch_b200 import weight_init as W
-    for kind, make, ref_fn, mine, inner in (('vit', _vit_image_checkpoint, ref.init_from_vit_pretrain_, W.remap_vit_checkpoint, 'state_dict'),
-                                            ('mae', _mae_checkpoint, ref.init_from_mae_pretrain_, W.remap_mae_checkpoint, 'model')):
-        path = str(tmp_path / f'{kind}.pth')
-        torch.save({inner: make()}, path)
-        catch = _Catch()
-        ref_fn(catch, path, conv_type, attention_type, copy_strategy, extend, 2, 1)
-        got = mine(make(), conv_type, attention_type, copy_strategy, extend, 2, 1)
-        assert sorted(got.keys()) == sorted(catch.got.keys()), kind
-        for k in got:
-            assert torch.equal(got[k], catch.got[k]), (kind, k)
-
-
-def test_kinetics_remap_equals_the_reference():
-    ref = _reference_weight_init()
-    from videotransformer_pytorch_b200 import weight_init as W
+def _kinetics_checkpoint():
     g = torch.Generator().manual_seed(2)
-    sd = {'model.cls_token': torch.randn(1, 1, 8, generator=g), 'model.a.attn.in_proj_weight': torch.randn(24, 8, generator=g),
-          'model.a.attn.out_proj.bias': torch.randn(8, generator=g), 'cls_head.cls_head.weight': torch.randn(4, 8, generator=g)}
-    theirs = dict(sd)
-    ref.replace_state_dict(theirs)
-    mine = W.remap_kinetics_checkpoint(sd)
-    assert sorted(mine) == sorted(theirs) and all(torch.equal(mine[k], theirs[k]) for k in mine)
+    return {'model.cls_token': torch.randn(1, 1, 8, generator=g), 'model.a.attn.in_proj_weight': torch.randn(24, 8, generator=g),
+            'model.a.attn.out_proj.bias': torch.randn(8, generator=g), 'cls_head.cls_head.weight': torch.randn(4, 8, generator=g)}
+
+
+@pytest.mark.parametrize('conv_type,attention_type,copy_strategy,extend', REMAP_CASES)
+def test_vit_and_mae_remaps_equal_the_reference(reference_remaps, conv_type, attention_type, copy_strategy, extend):
+    from videotransformer_pytorch_b200 import weight_init as W
+    for kind, make, mine in (('vit', _vit_image_checkpoint, W.remap_vit_checkpoint),
+                             ('mae', _mae_checkpoint, W.remap_mae_checkpoint)):
+        theirs = reference_remaps[remap_case_id(kind, conv_type, attention_type, copy_strategy, extend)]
+        got = state_digest(mine(make(), conv_type, attention_type, copy_strategy, extend, 2, 1))
+        assert sorted(got.keys()) == sorted(theirs.keys()), kind
+        for k in got:
+            assert got[k] == theirs[k], (kind, k)
+
+
+def test_kinetics_remap_equals_the_reference(reference_remaps):
+    from videotransformer_pytorch_b200 import weight_init as W
+    mine = state_digest(W.remap_kinetics_checkpoint(_kinetics_checkpoint()))
+    assert mine == reference_remaps['kinetics']
 
 
 def test_constructors_accept_pretrain_pth(tmp_path):

@@ -1,49 +1,37 @@
-"""The reference's UNMODIFIED model_trainer.py imported with the shim directory first on sys.path: its
-`from transformer import ...` / `from video_transformer import ...` / `from mixup import Mixup` resolve to this package,
-`VideoTransformer.__init__` (model_trainer.py:40-104) builds the B200 modules, and a forward runs (kernel table = CPU
-emulation).  Build-container only: needs /root/reference; its absent third-party imports (pytorch_lightning, torchmetrics,
-timm, matplotlib) are stubbed — none of them is on the hot path."""
+"""The shim directory stands in for the reference's top-level modules, so its unmodified model_trainer.py builds the B200
+modules.  What the reference asks of those modules is stored in tests/golden/reference_trainer.json (written by
+`oracle/make_golden.py reference_trainer` from the reference itself): the names its files import from them, the
+constructor calls `VideoTransformer.__init__` (model_trainer.py:40-104) makes, and the parameter surface of the trainer
+built from the reference's own modules.  Here those imports resolve through the shim, the recorded calls build the B200
+modules, and a forward + backward runs (kernel table = CPU emulation)."""
 import importlib
+import json
 import os
 import sys
-import types
 
 import pytest
 import torch
 
-REF = '/root/reference'
-SHIM = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'videotransformer_pytorch_b200', 'shim')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+SHIM = os.path.join(ROOT, 'videotransformer_pytorch_b200', 'shim')
+SHIM_MODULES = ('transformer', 'video_transformer', 'mixup', 'mask_generator')
+TRAINER_CFG = dict(objective='supervised', arch='timesformer', pretrain_pth=None, weights_from='imagenet', img_size=32,
+                   num_frames=2, attention_type='divided_space_time', num_class=5, eval_metrics='finetune', mixup=False)
 
 
 @pytest.fixture
 def reference_trainer():
-    if not os.path.isdir(REF):
-        pytest.skip('/root/reference not present (build container only)')
+    with open(os.path.join(ROOT, 'tests', 'golden', 'reference_trainer.json')) as fh:
+        return json.load(fh)
+
+
+@pytest.fixture
+def shim_modules():
     saved_path = list(sys.path)
-    saved_mods = {k: sys.modules.get(k) for k in ('transformer', 'video_transformer', 'mixup', 'mask_generator', 'model_trainer',
-                                                   'utils', 'optimizer', 'weight_init')}
-
-    def stub(name, **attrs):
-        m = types.ModuleType(name)
-        m.__dict__.update(attrs)
-        sys.modules[name] = m
-        return m
-
-    class Accuracy:
-        def __init__(self, *a, **k):
-            pass
-
-    pl = stub('pytorch_lightning', LightningModule=torch.nn.Module)
-    stub('pytorch_lightning.utilities')
-    stub('pytorch_lightning.utilities.distributed', rank_zero_only=lambda f: f)
-    stub('torchmetrics', Accuracy=Accuracy)
-    stub('timm'); stub('timm.loss', SoftTargetCrossEntropy=torch.nn.CrossEntropyLoss)
-    stub('matplotlib'); stub('matplotlib.pyplot')
-    for k in saved_mods:
-        sys.modules.pop(k, None)
-    sys.path[:0] = [SHIM, REF]
+    saved_mods = {k: sys.modules.pop(k, None) for k in SHIM_MODULES}
+    sys.path.insert(0, SHIM)
     try:
-        yield importlib.import_module('model_trainer')
+        yield {k: importlib.import_module(k) for k in SHIM_MODULES}
     finally:
         sys.path[:] = saved_path
         for k, v in saved_mods.items():
@@ -52,26 +40,37 @@ def reference_trainer():
                 sys.modules[k] = v
 
 
-def test_reference_trainer_builds_b200_modules_through_the_shim(reference_trainer, emu):
+def test_reference_trainer_builds_b200_modules_through_the_shim(reference_trainer, shim_modules, emu):
     import videotransformer_pytorch_b200 as pkg
-    mt = reference_trainer
-    assert mt.TimeSformer is pkg.TimeSformer and mt.ViViT is pkg.ViViT and mt.MaskFeat is pkg.MaskFeat
-    assert mt.ClassificationHead is pkg.ClassificationHead and mt.Mixup is pkg.Mixup
-    assert 'reference' in mt.__file__                      # the trainer itself is the reference's file, unmodified
-    cfg = types.SimpleNamespace(objective='supervised', arch='timesformer', pretrain_pth=None, weights_from='imagenet',
-                                img_size=32, num_frames=2, attention_type='divided_space_time', num_class=5,
-                                eval_metrics='finetune', mixup=False)
-    vt = mt.VideoTransformer(cfg, trainer=None, ckpt_dir='.', do_eval=False, do_test=False)
-    assert isinstance(vt.model, pkg.TimeSformer) and isinstance(vt.cls_head, pkg.ClassificationHead)
-    assert vt.no_weight_decay_keywords() == vt.model.no_weight_decay_keywords()
+    ref = reference_trainer
+    assert ref['cfg'] == TRAINER_CFG
+    # every name the reference imports from a shimmed module resolves, and the trainer's five are the package's classes
+    for mod, names in ref['imports'].items():
+        for name in names:
+            assert hasattr(shim_modules[mod], name), (mod, name)
+    vt, tr = shim_modules['video_transformer'], shim_modules['transformer']
+    assert vt.TimeSformer is pkg.TimeSformer and vt.ViViT is pkg.ViViT and vt.MaskFeat is pkg.MaskFeat
+    assert tr.ClassificationHead is pkg.ClassificationHead and shim_modules['mixup'].Mixup is pkg.Mixup
+    assert set(ref['imports']['video_transformer']) >= {'TimeSformer', 'ViViT', 'MaskFeat'}
+    assert 'ClassificationHead' in ref['imports']['transformer'] and 'Mixup' in ref['imports']['mixup']
+    # the constructor calls the reference trainer makes for this configuration, through the shim
+    built = {}
+    for name, args, kwargs in ref['constructions']:
+        built[name] = getattr(vt if hasattr(vt, name) else tr, name)(*args, **kwargs)
+    assert sorted(built) == ['ClassificationHead', 'TimeSformer']
+    trainer = torch.nn.Module()
+    trainer.model, trainer.cls_head = built['TimeSformer'], built['ClassificationHead']
+    assert isinstance(trainer.model, pkg.TimeSformer) and isinstance(trainer.cls_head, pkg.ClassificationHead)
+    assert sorted(ref['no_weight_decay_keywords']) == sorted(trainer.model.no_weight_decay_keywords())
+    # the parameter surface the reference's optimizer grouping walks (optimizer.py:49), name for name and shape for shape
+    assert [[n, list(p.shape)] for n, p in trainer.named_parameters()] == ref['named_parameters']
+    names = [n for n, _ in trainer.named_parameters()]
+    assert 'model.transformer_layers.layers.0.attentions.0.temporal_fc.weight' in names and 'cls_head.cls_head.weight' in names
     # the reference's training_step core (model_trainer.py:204-208) on a tiny clip; embed_dims 768 is fixed by the ctor
     x = torch.randn(2, 2, 3, 32, 32)
     y = torch.tensor([1, 3])
-    preds = vt.cls_head(vt.model(x))
-    loss = vt.loss_fn(preds, y)
+    preds = trainer.cls_head(trainer.model(x))
+    loss = torch.nn.CrossEntropyLoss()(preds, y)
     loss.backward()
     assert preds.shape == (2, 5) and torch.isfinite(loss)
-    assert all(p.grad is not None for p in vt.model.parameters())
-    # the reference's own optimizer grouping walks named_parameters() of these modules (optimizer.py:49)
-    names = [n for n, _ in vt.named_parameters()]
-    assert 'model.transformer_layers.layers.0.attentions.0.temporal_fc.weight' in names and 'cls_head.cls_head.weight' in names
+    assert all(p.grad is not None for p in trainer.model.parameters())
