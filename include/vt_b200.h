@@ -433,6 +433,23 @@ typedef struct {
 } vt_im2col_u8_mix_params;
 int vt_im2col_u8_mix_bf16(const vt_im2col_u8_mix_params* p, void* stream);
 
+/* Bicubic resampling of the spatial position table for inputs of another size than img_size
+ * (TimeSformer.interpolate_pos_encoding, video_transformer.py:171-191: F.interpolate(mode='bicubic', align_corners=False)
+ * with a scale factor).  Row 0 (cls) is copied; patch row 1 + i*src_side + j of the table is grid cell (i, j).
+ *   vt_pos_interp_fwd: in fp32 [1 + src_side^2, D] -> out fp32 [1 + out_rows*out_cols, D], output cell (i, j) at row
+ *                      1 + i*out_cols + j samples source coordinate ((i + 0.5) * scale_r - 0.5, (j + 0.5) * scale_c - 0.5)
+ *                      with the 4 x 4 cubic-convolution taps (A = -0.75) clamped to the grid.
+ *   vt_pos_interp_bwd: its adjoint, in = d out [1 + out_rows*out_cols, D] -> out = d table [1 + src_side^2, D]; gather
+ *                      form, deterministic.  (out_rows + out_cols) * src_side * 4 bytes must fit in 48 KB.
+ * scale_r / scale_c = (float)(1.0 / scale_factor) as ATen computes them for fp32 input.  D % 4 == 0, 16-byte aligned. */
+typedef struct {
+  const float* in; float* out;
+  int32_t D, src_side, out_rows, out_cols;
+  float scale_r, scale_c;
+} vt_pos_interp_params;
+int vt_pos_interp_fwd(const vt_pos_interp_params* p, void* stream);
+int vt_pos_interp_bwd(const vt_pos_interp_params* p, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -214,6 +214,11 @@ class Im2colU8MixParams(C.Structure):
                 ('C', c_i32), ('H', c_i32), ('W', c_i32), ('tube', c_i32), ('ph', c_i32), ('pw', c_i32)]
 
 
+class PosInterpParams(C.Structure):
+    _fields_ = [('inp', c_vp), ('out', c_vp), ('D', c_i32), ('src_side', c_i32), ('out_rows', c_i32), ('out_cols', c_i32),
+                ('scale_r', c_f32), ('scale_c', c_f32)]
+
+
 EXPORTS = ['vt_version', 'vt_last_error', 'vt_sm_count', 'vt_set_reserved_sms', 'vt_launch_count', 'vt_gemm', 'vt_layernorm_fwd', 'vt_ln_bwd_blocks',
            'vt_layernorm_bwd', 'vt_reduce_rows', 'vt_colsum_chunks', 'vt_colsum_bf16', 'vt_cast_f32_bf16',
            'vt_cls_rows', 'vt_gather_cast_colsum_blocks', 'vt_gather_cast_colsum_bf16', 'vt_gelu_bwd_colsum_blocks', 'vt_gelu_bwd_colsum_bf16',
@@ -222,7 +227,7 @@ EXPORTS = ['vt_version', 'vt_last_error', 'vt_sm_count', 'vt_set_reserved_sms', 
            'vt_maxpool_bwd', 'vt_im2col3d_bf16', 'vt_mvit_tokens_fwd', 'vt_mvit_tokens_bwd', 'vt_mse_blocks',
            'vt_mse_fwd', 'vt_mse_bwd', 'vt_opt_norm2', 'vt_opt_sgd', 'vt_opt_adamw',
            'vt_linear_small_fwd', 'vt_linear_small_bwd', 'vt_softmax_ce', 'vt_scale_by_scalar', 'vt_attn_probs',
-           'vt_im2col_u8_mix_bf16']
+           'vt_im2col_u8_mix_bf16', 'vt_pos_interp_fwd', 'vt_pos_interp_bwd']
 
 _dll = None
 
@@ -705,6 +710,32 @@ class CudaKernels:
         p.B, p.T, p.C, p.H, p.W, p.tube, p.ph, p.pw = B, T, Cc, H, W, tube, ph, pw
         _check(lib.vt_col2im_f32(C.byref(p), _stream()), 'vt_col2im_f32')
         return dx
+
+    # -- position-table resampling -------------------------------------------------------------
+    def _pos_interp(self, fn, src, rows_out, side, rows, cols, scale_r, scale_c):
+        lib = load_library()
+        src = _req(src, torch.float32, fn + '.in')
+        if src.dim() != 2 or not src.is_contiguous():
+            raise RuntimeError(f'{fn}: expected a contiguous [rows, D] table')
+        out = torch.empty((rows_out, src.shape[1]), dtype=torch.float32, device=src.device)
+        p = PosInterpParams()
+        p.inp, p.out = src.data_ptr(), out.data_ptr()
+        p.D, p.src_side, p.out_rows, p.out_cols = src.shape[1], side, rows, cols
+        p.scale_r, p.scale_c = scale_r, scale_c
+        _check(getattr(lib, fn)(C.byref(p), _stream()), fn)
+        return out
+
+    def pos_interp_fwd(self, table, side, rows, cols, scale_r, scale_c):
+        """fp32 [1 + side^2, D] -> bicubically resampled [1 + rows*cols, D] (cls row copied); scale_* = 1 / scale factor"""
+        if table.shape[0] != 1 + side * side:
+            raise RuntimeError(f'pos_interp_fwd: table has {table.shape[0]} rows, expected 1 + {side}^2')
+        return self._pos_interp('vt_pos_interp_fwd', table, 1 + rows * cols, side, rows, cols, scale_r, scale_c)
+
+    def pos_interp_bwd(self, dout, side, rows, cols, scale_r, scale_c):
+        """adjoint of pos_interp_fwd: fp32 [1 + rows*cols, D] -> [1 + side^2, D]"""
+        if dout.shape[0] != 1 + rows * cols:
+            raise RuntimeError(f'pos_interp_bwd: gradient has {dout.shape[0]} rows, expected 1 + {rows}*{cols}')
+        return self._pos_interp('vt_pos_interp_bwd', dout, 1 + side * side, side, rows, cols, scale_r, scale_c)
 
     # -- HOG ------------------------------------------------------------------------------------
     def hog(self, frames, lut, want_bins=False):

@@ -9,6 +9,7 @@ C-ABI kernel launches (see _lib.K):
   FFNFn           <- FFNWithPreNorm.forward                        (transformer.py:516-523)
   PatchTokensFn   <- PatchEmbed.forward + TimeSformer/ViViT.prepare_tokens
                      (transformer.py:138-151, video_transformer.py:193-240 / :455-475)
+  PosEmbedInterpFn <- TimeSformer.interpolate_pos_encoding's bicubic F.interpolate (video_transformer.py:171-191)
   ClsNormFn       <- final nn.LayerNorm(eps=1e-6) + cls select     (video_transformer.py:251-254)
   AttentionCoreFn <- Attention.forward (stand-alone use)            (transformer.py:165-177)
 
@@ -310,7 +311,13 @@ class SpatialAttnFn(torch.autograd.Function):
         hd = D // H
         xn, mean, rstd = k.ln_fwd(x2, ln_w, ln_b, eps, in_row=maps['sp_in'], rows=Ms)
         qkv = k.gemm(xn, qkv_wh, Ms, 3 * D, D, bias=qkv_b, epi='bf16', tag='qkv')
-        cx, lse, _ = k.attn_fwd(qkv, B * T, P + 1, H, hd, hd ** -0.5)
+        if P + 1 <= ATTN_SINGLE_PASS_MAX:
+            cx, lse, _ = k.attn_fwd(qkv, B * T, P + 1, H, hd, hd ** -0.5)
+        else:
+            # frames past 16 x 16 patches (img_size >= 256 at patch 16): streaming tcgen05 kernel, q/k/v read in place
+            q4, k4, v4 = _packed_heads(qkv, B * T, P + 1, H, hd)
+            cx, lse = k.xattn_fwd(q4, k4, v4, hd ** -0.5)
+            cx = cx.view(Ms, D)
         ybig = torch.empty((R + B * T, D), dtype=torch.float32, device=x.device)
         k.gemm(cx, proj_wh, Ms, D, D, bias=proj_b, epi='f32', aux=x2, aux_row=maps['sp_aux'], out=ybig,
                out_row=maps['sp_out'], row_scale=dp, row_map=affine_row_maps(B, T, P, D)['spatial'], tag='proj')
@@ -335,7 +342,10 @@ class SpatialAttnFn(torch.autograd.Function):
         g, d_proj_b = _cast_with_colsum(k, dy2, in_row=maps['sp_in'], row_scale=_mul_opt(dp, maps['sp_cls_scale']), rows=Ms)
         d_proj_w = _wgrad(g, cx, D, D, Ms, tag='proj', wptr=ctx.wptrs[1])
         dcx = _dgrad(g, proj_wh, Ms, D, D, epi='bf16', tag='proj')
-        dqkv = k.attn_bwd(qkv, cx, dcx, lse, B * T, P + 1, H, hd, hd ** -0.5)
+        if P + 1 <= ATTN_SINGLE_PASS_MAX:
+            dqkv = k.attn_bwd(qkv, cx, dcx, lse, B * T, P + 1, H, hd, hd ** -0.5)
+        else:
+            dqkv = _streaming_attn_bwd(k, qkv, cx, dcx, lse, B * T, P + 1, H, hd)
         d_qkv_w = _wgrad(dqkv, xn, 3 * D, D, Ms, tag='qkv', wptr=ctx.wptrs[0])
         d_qkv_b = k.colsum(dqkv)
         dxn = _dgrad(dqkv, qkv_wh, Ms, D, 3 * D, epi='bf16', tag='qkv')
@@ -534,6 +544,26 @@ class PatchTokensFn(torch.autograd.Function):
             dx = k.col2im(dcols, xshape, tube, wshape[-2], wshape[-1])
         # small grads are returned as fresh contiguous tensors (not views) so autograd can adopt them in place
         return dx, dw.contiguous(), db, dcls.reshape(cshape).clone(), dpos.contiguous(), dtime, None, None, None, None, None
+
+
+# --------------------------------------------------------------------------------------------------
+class PosEmbedInterpFn(torch.autograd.Function):
+    """Bicubic resampling of the spatial position table [1, 1+side^2, D] -> [1, 1+rows*cols, D] (cls row copied), the
+    F.interpolate of TimeSformer.interpolate_pos_encoding (video_transformer.py:184-191); scale_r / scale_c are the inverse
+    scale factors.  Backward is the kernel's adjoint."""
+
+    @staticmethod
+    def forward(ctx, pos, side, rows, cols, scale_r, scale_c):
+        D = pos.shape[-1]
+        out = K().pos_interp_fwd(pos.reshape(-1, D).float().contiguous(), side, rows, cols, scale_r, scale_c)
+        ctx.geom = (tuple(pos.shape), side, rows, cols, scale_r, scale_c)
+        return out.view(1, 1 + rows * cols, D)
+
+    @staticmethod
+    def backward(ctx, dout):
+        pshape, side, rows, cols, scale_r, scale_c = ctx.geom
+        d = K().pos_interp_bwd(dout.reshape(-1, pshape[-1]).float().contiguous(), side, rows, cols, scale_r, scale_c)
+        return d.view(pshape), None, None, None, None, None
 
 
 # --------------------------------------------------------------------------------------------------

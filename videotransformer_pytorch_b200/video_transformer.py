@@ -9,6 +9,8 @@ PyTorch.
 """
 from __future__ import annotations
 
+import math
+
 import torch
 import torch.nn as nn
 
@@ -124,11 +126,29 @@ class TimeSformer(_ByteClipInput, nn.Module):
         return {'pos_embed', 'cls_token', 'mask_token'}
 
     def interpolate_pos_encoding(self, x, w, h):
-        npatch = x.shape[1] - 1
-        N = self.pos_embed.shape[1] - 1
+        """reference video_transformer.py:171-191: the spatial position table for tokens `x` ([*, 1 + npatch, D], cls
+        first) of a clip of width w and height h — pos_embed itself when the grid is the model's own, else its patch rows
+        resampled bicubically (F.interpolate with scale factors (w//p + 0.1) / sqrt(N), (h//p + 0.1) / sqrt(N)) on the
+        device.  As in the reference the result has w//p rows and h//p columns, flattened row-major: for w != h it is
+        added to tokens in (h//p, w//p) raster order, i.e. transposed.  Reproduced, not fixed."""
+        pos = self.pos_embed if self.use_learnable_pos_emb else self.pos_embed.to(x.device).detach()
+        return self._resampled_pos(pos, x.shape[1] - 1, w, h)
+
+    def _resampled_pos(self, pos, npatch, w, h):
+        N = pos.shape[1] - 1
         if npatch == N and w == h:
-            return self.pos_embed
-        raise NotImplementedError('bicubic pos-embed interpolation (img_size != training size) is outside the hot path')
+            return pos
+        gh, gw = (s // p for s, p in zip(self.patch_embed.img_size, self.patch_embed.patch_size))
+        if gh != gw:
+            raise NotImplementedError(f'pos_embed interpolation needs a square patch grid; this model has {gh} x {gw} '
+                                      f'patches (img_size {self.patch_embed.img_size}), so it only takes clips of that size')
+        p = self.patch_embed.patch_size[0]
+        sq = math.sqrt(N)
+        sf_r, sf_c = (w // p + 0.1) / sq, (h // p + 0.1) / sq          # the `+ 0.1` of the reference (:183)
+        rows, cols = math.floor(gh * sf_r), math.floor(gh * sf_c)      # F.interpolate's output size for a scale factor
+        assert (rows, cols) == (w // p, h // p), (rows, cols, w, h)
+        # ATen samples at (dst + 0.5) / scale_factor - 0.5 with 1 / scale_factor taken in double, then cast to float
+        return ops.PosEmbedInterpFn.apply(pos, gh, rows, cols, 1.0 / sf_r, 1.0 / sf_c)
 
     def _embeds(self, x):
         pos = self.pos_embed
@@ -144,11 +164,13 @@ class TimeSformer(_ByteClipInput, nn.Module):
             b, t, h, w, c = x.shape
         else:
             b, t, c, h, w = x.shape
-        P = self.patch_embed.num_patches
-        if (h // self.patch_embed.patch_size[0]) * (w // self.patch_embed.patch_size[1]) != P or w != h:
-            raise NotImplementedError('input size must match img_size (no pos-embed interpolation on the hot path)')
-        pos, tim = self._embeds(x)
         pe = self.patch_embed
+        ph, pw = pe.projection.kernel_size
+        if h % ph or w % pw or pw % 8:
+            raise NotImplementedError(f'input {h} x {w}: the patch kernels need H % {ph} == 0, W % {pw} == 0 and a patch '
+                                      f'width that is a multiple of 8 (patch {ph} x {pw})')
+        pos, tim = self._embeds(x)
+        pos = self._resampled_pos(pos, (h // ph) * (w // pw), w, h)
         mode = 'frames' if self.attention_type == 'space_only' else 'timesformer'   # space_only: per-frame tokens
         tok = ops.PatchTokensFn.apply(x, _f32(pe.projection.weight), _f32(pe.projection.bias), self.cls_token, pos, tim,
                                       pe.shadow(), mode, 1, norm, plan)
@@ -257,8 +279,12 @@ class ViViT(_ByteClipInput, nn.Module):
     def prepare_tokens(self, x):
         x, norm, plan = self._unwrap_clip(x)
         b = x.shape[0]
-        pos = self.pos_embed if self.use_learnable_pos_emb else self.pos_embed.to(x.device).detach()
+        h, w = x.shape[2:4] if norm is not None else x.shape[3:5]
         pe = self.patch_embed
+        if (h // pe.patch_size[0]) * (w // pe.patch_size[1]) != pe.num_patches:
+            raise NotImplementedError(f'ViViT takes clips of img_size {pe.img_size} only (got {h} x {w}): like the reference '
+                                      f'it adds pos_embed without interpolation')
+        pos = self.pos_embed if self.use_learnable_pos_emb else self.pos_embed.to(x.device).detach()
         if self.attention_type == 'fact_encoder':
             tok = ops.PatchTokensFn.apply(x, _f32(pe.projection.weight), _f32(pe.projection.bias), self.cls_token, pos, None,
                                           pe.shadow(), 'frames', self.tube_size, norm, plan)
